@@ -5,20 +5,25 @@ synthetic 512x512x16 video, grid_size=80 (N=6400 tracks), 6 refinement iteration
     python bench.py --gpus 1 --steps 5 --warmup 3                 # this repo (libct3_b200.so on the B200)
     python bench.py --impl reference --gpus 1 --steps 2 --warmup 1  # CPU arm: the UNMODIFIED reference on the host cores
     python bench.py --grid 30 | --frames 48 | --online --grid 50    # BASELINE.json configs C2 / C3 / C4
+    python bench.py --dump-outputs DIR                              # + the last timed step's outputs as DIR/*.npy
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W                    # N replicas, one clip per GPU (weak scaling)
 
-One JSON line on stdout (rank 0).  A "step" = one CoTrackerPredictor.forward over one clip.
+One JSON line on stdout (rank 0).  A "step" = one CoTrackerPredictor.forward over one clip; --steps K times exactly K.
   value : whole-job points*frames/s with the clip resident in HBM when the timed region starts
   e2e   : same call with the clip in pinned HOST memory (H2D copy + D2H of tracks/visibility inside the region)
   roofline     : dominant kernel (the tcgen05 split-bf16x3 GEMM) -- algorithmic FLOPs / live CUDA-event time
   roofline_corr: the fused sampling+correlation kernel against the HBM roofline (4.71 GB/iteration, SURVEY 8d)
   cpu_baseline : the reference's own PyTorch-CPU path on a bounded sample of the same workload (rank 0, N=1 only)
 
-CPU arm: the unmodified reference package is looked up in $COTRACKER_REFERENCE, /root/reference (build container)
-and baseline/_ref (pip --target install of the reference, travels to the GPU box; DESIGN.md section 5) and driven
-through its own CoTrackerPredictor with the shared seeded state dict ("kind": "reference").  Only when none of
-them exists does the arm fall back to the oracle port ("kind": "port").
+--dump-outputs DIR writes what the last timed step (the `value` path) returned on rank 0, tracks.npy and
+visibility.npy (float32, visibility as 0/1), so that two builds can be compared output for output: inputs and weights
+are seeded, so the same arguments give the same inputs.  Above 64 MB in all, a fixed seeded sample of the tracks is
+written instead, with their indices as track_sample.npy.
+
+CPU arm: the unmodified reference package is looked up in $COTRACKER_REFERENCE and baseline/_ref (pip --target
+install of the reference; DESIGN.md section 5) and driven through its own CoTrackerPredictor with the shared seeded
+state dict ("kind": "reference").  Only when neither exists does the arm fall back to the oracle port ("kind": "port").
 Synthetic clip: cotracker_b200.synthetic.texture_video (integer-valued random texture, nearest-upsampled x8,
 translated per frame) -- NOT BASELINE.md section 3's bicubic recipe: integer-only construction is bit-identical
 on every machine, which the committed full-size goldens (tests/golden/headline_grid80*.npz) rely on.
@@ -34,6 +39,7 @@ import sys
 import tempfile
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -73,7 +79,7 @@ def usable_cores() -> int:
 
 def find_reference():
     """Directory holding the unmodified reference package (`cotracker/predictor.py`), or None."""
-    for p in (os.environ.get("COTRACKER_REFERENCE"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
+    for p in (os.environ.get("COTRACKER_REFERENCE"), os.path.join(ROOT, "baseline", "_ref")):
         if p and os.path.isfile(os.path.join(p, "cotracker", "predictor.py")):
             return p
     return None
@@ -185,7 +191,7 @@ def cpu_run(sd, video, G, online, ref_dir):
 def bench_reference(args, rank):
     """CPU arm: the reference's own PyTorch-CPU implementation on all usable host cores, on the SAME config as the
     B200 arm (grid/frames as given; default = the headline shape).  One repetition takes 1-2 minutes there, so the
-    warm-up runs at grid_size=10 and the timed repetitions are capped by a time budget; `steps` is what actually ran."""
+    warm-up runs at grid_size=10; the timed repetitions are exactly `steps`."""
     if rank != 0:
         return
     from cotracker_b200.synthetic import seeded_state_dict, texture_video
@@ -198,11 +204,7 @@ def bench_reference(args, rank):
     video = texture_video(T, SIZE, SIZE, seed=0)
     for _ in range(min(args.warmup, 1)):
         cpu_run(sd, video, 10, online, ref_dir)            # thread pool, allocator, oneDNN primitive caches
-    budget_s, times = 240.0, []
-    while len(times) < max(args.steps, 1):
-        times.append(cpu_run(sd, video, G, online, ref_dir))
-        if sum(times) + times[-1] > budget_s:
-            break
+    times = [cpu_run(sd, video, G, online, ref_dir) for _ in range(args.steps)]
     ms = 1e3 * sum(times) / len(times)
     units = G * G * (8 if online else T)
     value = units / (ms / 1e3)
@@ -221,6 +223,24 @@ def bench_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT = 64 * 10**6 - 4096     # bytes of array data: 64 MB in all with the .npy headers
+
+
+def dump_outputs(out_dir, outputs):
+    """outputs: name -> [B, T, N, ...] tensor of one predictor call; written as out_dir/<name>.npy in float32.  Above
+    DUMP_LIMIT bytes in all, only a fixed seeded sample of the N tracks is written, its indices as track_sample.npy."""
+    outputs = {k: v.float().cpu() for k, v in outputs.items()}
+    n = outputs["tracks"].shape[2]
+    per_track = sum(v.numel() * 4 for v in outputs.values()) // n + 8
+    if per_track * n > DUMP_LIMIT:
+        keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_LIMIT // per_track].sort().values
+        outputs = {k: v[:, :, keep] for k, v in outputs.items()}
+        outputs["track_sample"] = keep.double()
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in outputs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.numpy())
+
+
 # ---------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -234,7 +254,13 @@ def main():
     ap.add_argument("--online", action="store_true", help="BASELINE config C4: cotracker3_online, window 16 / step 8")
     ap.add_argument("--opt", action="append", default=[], metavar="NAME=VALUE",
                     help="library option for A/B runs, e.g. --opt fuse=1 --opt prec.fc1=2 (ct3_set_option)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's tracks and visibility to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -338,8 +364,10 @@ def main():
         run_resident()
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ms_step, _ = timed(run_resident, args.steps)
+    ms_step, last = timed(run_resident, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"tracks": last[0], "visibility": last[1]})
     for _ in range(1):
         run_e2e()
     ms_e2e, (tr, vis) = timed(run_e2e, args.steps)

@@ -1,16 +1,19 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference) on seeded
-weights and seeded synthetic inputs.  Run in the build container only (the GPU box has no /root/reference):
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (a facebookresearch/co-tracker checkout, given as
+$COTRACKER_REFERENCE) on seeded weights and seeded synthetic inputs.  The tests only read the stored files:
 
-    python oracle/make_golden.py                 # every case (the BASELINE-scale ones take minutes each)
-    python oracle/make_golden.py c2_grid30 ...   # selected cases
+    COTRACKER_REFERENCE=<checkout> python oracle/make_golden.py                 # every golden (minutes each for
+                                                                                # the BASELINE-scale cases)
+    COTRACKER_REFERENCE=<checkout> python oracle/make_golden.py c2_grid30 ...   # selected ones
 
 Only the *outputs* are stored (tiny); weights and inputs are re-created from their seeds by
 cotracker_b200.synthetic on whichever machine runs the tests (the one real clip, BASELINE.json config 1's
-assets/apple.mp4, travels as a 120x216 area-downsampled uint8 copy of its 50 decoded frames:
-tests/golden/apple_frames_120x216.npz, made by `make_apple_fixture()` below).  Cases are listed in CASES below
+assets/apple.mp4, travels as a 60x108 area-downsampled uint8 copy of its 50 decoded frames:
+tests/golden/apple_frames_60x108.npz, made by `make_apple_fixture()` below).  Cases are listed in CASES below
 and are the single source of truth for tests/test_golden*.py.  Predictor cases also store the model's visibility
 (and confidence) probabilities -- captured with a forward hook on the unmodified reference model -- so a test
-can tell a genuine visibility mismatch from a value sitting on the threshold.
+can tell a genuine visibility mismatch from a value sitting on the threshold.  Every golden file stays below 1 MB:
+a case whose full output would not keeps a fixed, seeded sample of its tracks (TRACK_SAMPLE), and the stage-level
+golden (`reference_units`, make_unit_golden) keeps every k-th element of its larger arrays (`thin`).
 """
 from __future__ import annotations
 
@@ -22,9 +25,19 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = os.environ.get("COTRACKER_REFERENCE", "/root/reference")
 
 from cotracker_b200.synthetic import random_queries, seeded_state_dict, texture_video  # noqa: E402
+
+
+def reference_dir():
+    """The reference checkout named by $COTRACKER_REFERENCE, put first on sys.path (generation only)."""
+    ref = os.environ.get("COTRACKER_REFERENCE", "")
+    if not os.path.isfile(os.path.join(ref, "cotracker", "predictor.py")):
+        raise SystemExit("set COTRACKER_REFERENCE to a facebookresearch/co-tracker checkout")
+    if ref not in sys.path:
+        sys.path.insert(0, ref)
+    return ref
+
 
 # name -> config.  kind: model_offline | model_online_stream | model_online_slide | predictor_offline | predictor_online
 CASES = {
@@ -88,18 +101,32 @@ CASES = {
     "c4_online_grid50": dict(kind="predictor_online", T=40, H=512, W=512, grid=50, iters=6, wseed=1234, vseed=0,
                              head_gain=5.0, vis_gain=30.0, window_len=16),
 }
-APPLE_FIXTURE = os.path.join(ROOT, "tests", "golden", "apple_frames_120x216.npz")
+APPLE_FIXTURE = os.path.join(ROOT, "tests", "golden", "apple_frames_60x108.npz")
+
+# tracks kept in the golden of a case whose full output would exceed 1 MB (C4: 4 steps x up to 40 frames x 2500 tracks)
+TRACK_SAMPLE = {"c4_online_grid50": 640}
+
+
+def track_sample(name, n):
+    """The fixed, seeded, sorted subset of the n tracks that the golden of `name` keeps."""
+    g = torch.Generator().manual_seed(0)
+    return torch.randperm(n, generator=g)[:TRACK_SAMPLE[name]].sort().values
+
+
+def take_tracks(out, idx):
+    """Every output of a predictor case restricted to the tracks `idx` (axis 2 of tracks, visibility, probabilities)."""
+    return {k: v[:, :, idx] for k, v in out.items()}
 
 
 def make_apple_fixture():
-    """Decode assets/apple.mp4 (BASELINE.json config 1) and store an area-downsampled uint8 copy (build box only)."""
+    """Decode assets/apple.mp4 (BASELINE.json config 1) and store an area-downsampled uint8 copy."""
     import cv2
-    cap, frames = cv2.VideoCapture(os.path.join(REF, "assets", "apple.mp4")), []
+    cap, frames = cv2.VideoCapture(os.path.join(reference_dir(), "assets", "apple.mp4")), []
     while True:
         ok, f = cap.read()
         if not ok:
             break
-        frames.append(cv2.resize(cv2.cvtColor(f, cv2.COLOR_BGR2RGB), (216, 120), interpolation=cv2.INTER_AREA))
+        frames.append(cv2.resize(cv2.cvtColor(f, cv2.COLOR_BGR2RGB), (108, 60), interpolation=cv2.INTER_AREA))
     np.savez_compressed(APPLE_FIXTURE, frames=np.stack(frames))
 
 
@@ -162,7 +189,7 @@ def record_model_outputs(model):
 
 
 def run_reference(cfg):
-    sys.path.insert(0, REF)
+    reference_dir()
     from cotracker.models.build_cotracker import build_cotracker
     from cotracker.predictor import CoTrackerOnlinePredictor, CoTrackerPredictor
 
@@ -225,7 +252,7 @@ def eval_case_inputs():
 
 def make_eval_golden():
     """reference cotracker/models/evaluation_predictor.py:25-199, single-point (TAP-Vid protocol) and joint mode."""
-    sys.path.insert(0, REF)
+    reference_dir()
     from cotracker.models.build_cotracker import build_cotracker
     from cotracker.models.evaluation_predictor import EvaluationPredictor
     sd, video, queries = eval_case_inputs()
@@ -241,20 +268,116 @@ def make_eval_golden():
     print("eval_predictor", {k: v.shape for k, v in out.items()})
 
 
+THIN = 13   # odd and prime to every axis length below: the kept elements cover every row and every channel
+
+
+def thin(t):
+    """Every THIN-th element of `t`, flattened: what reference_units.npz keeps of an array larger than a few KB."""
+    return t.reshape(-1)[::THIN]
+
+
+UNIT_TIME_LENGTHS = (60, 16, 7)     # time-embedding lengths: the stored 60, and two interpolations of it
+UNIT_GRID_SIZES = (1, 5, 30)
+UNIT_SINCOS_LENGTHS = (16, 60)
+CENTRED_GRIDS = ((8, (50, 50), (120.5, 77.25)), (5, (384, 512), None), (1, (384, 512), None))
+
+
+def unit_inputs():
+    """Seeded weights and inputs of the stage-level golden (reference_units.npz; tests/test_oracle_vs_reference.py).
+    Amplified heads and correlation volumes x10 reach the regimes where end-to-end parity is blind (e.g. erf vs tanh
+    GELU in corr_mlp, SURVEY Appendix A)."""
+    sd = seeded_state_dict(2024, offline=True, window_len=60, head_gain=10.0, vis_gain=100.0)
+    x = {"updateformer": torch.randn(1, 33, 7, 1110, generator=torch.Generator().manual_seed(1)) * 2}
+    g = torch.Generator().manual_seed(2)
+    T, N, H, W = 3, 11, 12, 16
+    x["corr_fmap"] = torch.randn(1, T, 128, H, W, generator=g)
+    x["corr_coords"] = torch.rand(T, N, 2, generator=g) * torch.tensor([W + 4.0, H + 4.0]) - 2.0   # some outside
+    x["corr_support"] = torch.randn(1, 49, N, 128, generator=g)
+    x["corr_mlp_in"] = torch.randn(T, N, 2401, generator=g) * 10.0     # x10: where erf and tanh GELU differ
+    g = torch.Generator().manual_seed(3)
+    T, N, H, W = 4, 9, 12, 16
+    x["sup_fmap"] = torch.randn(1, T, 128, H, W, generator=g)
+    x["sup_qf"] = torch.randint(0, T, (1, N), generator=g)
+    x["sup_qc"] = torch.rand(1, N, 2, generator=g) * torch.tensor([W - 1.0, H - 1.0])
+    x["posenc"] = torch.randn(5, 3, 4, generator=torch.Generator().manual_seed(4)) * 0.1
+    x["encoder"] = texture_video(2, 64, 96, seed=5)[0] / 255 * 2 - 1
+    x["video"] = texture_video(5, 64, 96, seed=6)
+    x["queries"] = random_queries(9, 5, 64, 96, seed=7)
+    return sd, x
+
+
+def tapvid_problem(seed, b=2, n=17, t=11):
+    """Seeded TAP-Vid metric inputs (query_points, gt_occluded, gt_tracks, pred_occluded, pred_tracks)."""
+    r = np.random.default_rng(seed)
+    q = np.concatenate([r.integers(0, t, (b, n, 1)).astype(np.float64), r.uniform(0, 256, (b, n, 2))], axis=-1)
+    gt = r.uniform(0, 256, (b, n, t, 2))
+    pred = gt + r.normal(0, 3.0, gt.shape) * (r.uniform(size=(b, n, t, 1)) < 0.7)
+    occ = r.uniform(size=(b, n, t)) < 0.3
+    pocc = occ ^ (r.uniform(size=(b, n, t)) < 0.2)
+    return q, occ, gt, pocc, pred
+
+
+def make_unit_golden():
+    """Stage by stage, the reference on unit_inputs(), plus its query grids, sin-cos embeddings and TAP-Vid metrics."""
+    reference_dir()
+    from cotracker.evaluation.core.eval_utils import compute_tapvid_metrics
+    from cotracker.models.build_cotracker import build_cotracker
+    from cotracker.models.core.cotracker.cotracker3_online import posenc
+    from cotracker.models.core.embeddings import get_1d_sincos_pos_embed_from_grid
+    from cotracker.models.core.model_utils import get_points_on_a_grid
+    sd, x = unit_inputs()
+    m = build_cotracker(None, offline=True, window_len=60).eval()
+    m.load_state_dict(sd)
+    out = {}
+    with torch.no_grad():
+        out["updateformer"] = thin(m.updateformer(x["updateformer"]))
+        N = x["corr_coords"].shape[1]
+        feat = m.get_correlation_feat(x["corr_fmap"], x["corr_coords"])
+        s = x["corr_support"].view(1, 1, 7, 7, N, 128).squeeze(1).permute(0, 3, 1, 2, 4)
+        out["corr_volume"] = thin(torch.einsum("btnhwc,bnijc->btnhwij", feat, s))
+        out["corr_mlp"] = thin(m.corr_mlp(x["corr_mlp_in"]))
+        out["support"] = thin(m.get_track_feat(x["sup_fmap"], x["sup_qf"], x["sup_qc"], support_radius=3)[1][0])
+        out["posenc"] = posenc(x["posenc"], 0, 10)
+        for t in UNIT_TIME_LENGTHS:
+            out[f"time_embed{t}"] = thin(m.interpolate_time_embed(torch.zeros(1, t, 1110), t))
+        out["encoder"] = thin(m.fnet(x["encoder"]))
+        out["coords"], out["vis"], _, _ = m(x["video"], x["queries"], iters=3)
+    for size in UNIT_GRID_SIZES:
+        out[f"grid{size}"] = get_points_on_a_grid(size, (384, 512))
+    for L in UNIT_SINCOS_LENGTHS:
+        pos = torch.linspace(0, L - 1, L).reshape(1, L, 1)[0]
+        out[f"sincos{L}"] = thin(get_1d_sincos_pos_embed_from_grid(1110, pos))
+    for i, (size, extent, centre) in enumerate(CENTRED_GRIDS):
+        out[f"centred_grid{i}"] = get_points_on_a_grid(size, extent, centre)
+    for mode in ("first", "strided"):
+        for seed in range(4):
+            for k, v in compute_tapvid_metrics(*tapvid_problem(seed), mode).items():
+                out[f"tapvid_{mode}{seed}_{k}"] = v
+    path = os.path.join(ROOT, "tests", "golden", "reference_units.npz")
+    np.savez_compressed(path, **{k: np.asarray(v) for k, v in out.items()})
+    print("reference_units", len(out), "arrays", os.path.getsize(path), "bytes")
+
+
 def main():
     import time
     os.makedirs(os.path.join(ROOT, "tests", "golden"), exist_ok=True)
     if not os.path.exists(APPLE_FIXTURE):
         make_apple_fixture()
-    names = sys.argv[1:] or (list(CASES) + ["eval_predictor"])
+    names = sys.argv[1:] or (list(CASES) + ["eval_predictor", "reference_units"])
     if "eval_predictor" in names:
         names.remove("eval_predictor")
         make_eval_golden()
+    if "reference_units" in names:
+        names.remove("reference_units")
+        make_unit_golden()
     for name in names:
         cfg = CASES[name]
         t0 = time.perf_counter()
         out = run_reference(cfg)
         print(f"{name}: reference ran {time.perf_counter() - t0:.1f} s")
+        if name in TRACK_SAMPLE:
+            idx = track_sample(name, out[next(iter(out))].shape[2]).numpy()
+            out = dict(take_tracks(out, idx), track_sample=idx)
         path = os.path.join(ROOT, "tests", "golden", name + ".npz")
         np.savez_compressed(path, **out)
         print(name, {k: v.shape for k, v in out.items()}, os.path.getsize(path), "bytes")

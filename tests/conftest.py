@@ -13,15 +13,6 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
-@pytest.fixture(scope="session")
-def reference_path():
-    """Path of the unmodified reference checkout (build container only)."""
-    p = os.environ.get("COTRACKER_REFERENCE", "/root/reference")
-    if not os.path.isdir(os.path.join(p, "cotracker")):
-        pytest.skip("reference checkout not present on this machine")
-    return p
-
-
 # product defaults of the per-thread library options (api.cu); a test that changes one must put it back
 OPTION_DEFAULTS = {"gemm": 0, "corr": 0, "attn": 0, "prec.corr": 2, "prec.fc1": 3, "fuse": 1}
 

@@ -1,26 +1,17 @@
-"""Evaluation harness (SURVEY 8(f4)): the numpy TAP-Vid metrics against the LIVE reference implementation (build
-container) and, on the GPU, EvaluationPredictor against the reference's EvaluationPredictor output pinned in a golden."""
-import sys
-
+"""Evaluation harness (SURVEY 8(f4)): the numpy TAP-Vid metrics against the reference implementation's results
+(pinned in tests/golden/reference_units.npz) and, on the GPU, EvaluationPredictor against the reference's
+EvaluationPredictor output pinned in a golden."""
 import numpy as np
 import pytest
 import torch
 
+from cases import load_golden
 from cotracker_b200.evaluation import EvaluationPredictor, points_on_a_grid, tapvid_metrics
-
-
-def _random_problem(seed, b=2, n=17, t=11):
-    r = np.random.default_rng(seed)
-    q = np.concatenate([r.integers(0, t, (b, n, 1)).astype(np.float64), r.uniform(0, 256, (b, n, 2))], axis=-1)
-    gt = r.uniform(0, 256, (b, n, t, 2))
-    pred = gt + r.normal(0, 3.0, gt.shape) * (r.uniform(size=(b, n, t, 1)) < 0.7)
-    occ = r.uniform(size=(b, n, t)) < 0.3
-    pocc = occ ^ (r.uniform(size=(b, n, t)) < 0.2)
-    return q, occ, gt, pocc, pred
+from oracle.make_golden import CENTRED_GRIDS, tapvid_problem
 
 
 def test_perfect_prediction_scores_one():
-    q, occ, gt, _, _ = _random_problem(0)
+    q, occ, gt, _, _ = tapvid_problem(0)
     m = tapvid_metrics(q, occ, gt, occ, gt, "strided")
     assert np.allclose(m["average_jaccard"], 1.0) and np.allclose(m["average_pts_within_thresh"], 1.0)
     assert np.isclose(m["occlusion_accuracy"].sum(), 1.0)      # the reference normalises by the batch total
@@ -41,23 +32,21 @@ def test_hand_computed_case():
 
 
 @pytest.mark.parametrize("mode", ["first", "strided"])
-def test_metrics_match_live_reference(reference_path, mode):
-    sys.path.insert(0, reference_path)
-    from cotracker.evaluation.core.eval_utils import compute_tapvid_metrics
+def test_metrics_match_live_reference(mode):
+    ref = load_golden("reference_units")
     for seed in range(4):
-        args = _random_problem(seed)
-        want = compute_tapvid_metrics(*args, mode)
-        got = tapvid_metrics(*args, mode)
+        prefix = f"tapvid_{mode}{seed}_"
+        want = {k[len(prefix):]: v.numpy() for k, v in ref.items() if k.startswith(prefix)}
+        got = tapvid_metrics(*tapvid_problem(seed), mode)
         assert set(want) == set(got)
         for k in want:
             assert np.allclose(got[k], want[k], rtol=0, atol=1e-12), k
 
 
-def test_grid_with_centre_matches_live_reference(reference_path):
-    sys.path.insert(0, reference_path)
-    from cotracker.models.core.model_utils import get_points_on_a_grid
-    for size, extent, centre in ((8, (50, 50), (120.5, 77.25)), (5, (384, 512), None), (1, (384, 512), None)):
-        assert torch.equal(points_on_a_grid(size, extent, centre), get_points_on_a_grid(size, extent, centre))
+def test_grid_with_centre_matches_live_reference():
+    ref = load_golden("reference_units")
+    for i, (size, extent, centre) in enumerate(CENTRED_GRIDS):
+        assert torch.equal(points_on_a_grid(size, extent, centre), ref[f"centred_grid{i}"])
 
 
 @pytest.mark.gpu

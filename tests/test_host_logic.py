@@ -80,17 +80,17 @@ def test_grid_queries_match_reference_contract():
     assert get_points_on_a_grid(1, (384, 512)).tolist() == [[[256.0, 192.0]]]
 
 
-def test_grid_and_time_embedding_match_live_reference(reference_path):
-    sys.path.insert(0, reference_path)
-    from cotracker.models.core.model_utils import get_points_on_a_grid as ref_grid
-    from cotracker.models.core.embeddings import get_1d_sincos_pos_embed_from_grid
+def test_grid_and_time_embedding_match_live_reference():
+    """Query grids and sin-cos time embeddings against the reference's (pinned in tests/golden/reference_units.npz)."""
+    from cases import load_golden
     from cotracker_b200.model import sincos_time_embedding
     from cotracker_b200.predictor import get_points_on_a_grid
-    for size in (1, 5, 30):
-        assert torch.equal(get_points_on_a_grid(size, (384, 512)), ref_grid(size, (384, 512)))
-    for L in (16, 60):
-        ref = get_1d_sincos_pos_embed_from_grid(1110, torch.linspace(0, L - 1, L).reshape(1, L, 1)[0])
-        assert torch.equal(sincos_time_embedding(1110, L), ref)
+    from oracle.make_golden import UNIT_GRID_SIZES, UNIT_SINCOS_LENGTHS, thin
+    ref = load_golden("reference_units")
+    for size in UNIT_GRID_SIZES:
+        assert torch.equal(get_points_on_a_grid(size, (384, 512)), ref[f"grid{size}"])
+    for L in UNIT_SINCOS_LENGTHS:
+        assert torch.equal(thin(sincos_time_embedding(1110, L)), ref[f"sincos{L}"])
 
 
 def test_shard_clips():

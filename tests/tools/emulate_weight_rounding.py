@@ -1,4 +1,4 @@
-"""CPU emulation (reference model, this container only): what would a 2-product transformer GEMM cost in track error?
+"""CPU emulation (reference model, $COTRACKER_REFERENCE): what would a 2-product transformer GEMM cost in track error?
 
 A 2-product GEMM on fp16 planes keeps the activation exact to ~2^-22 (hi + lo) and rounds the WEIGHT to one fp16 plane
 (2^-12).  That is exactly the unmodified reference run with its transformer weights rounded to fp16, so the error of
@@ -51,6 +51,8 @@ def main():
         finally:
             mg.seeded_state_dict = orig
         with np.load(os.path.join(ROOT, "tests", "golden", name + ".npz")) as z:
+            if "track_sample" in z.files:
+                got = mg.take_tracks(got, z["track_sample"])
             worst, flips = 0.0, 0
             for k in got:
                 if k.startswith("tracks") or k.startswith("coords"):
